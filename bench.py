@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the PINN training hot path (BASELINE.json metric: collocation-points/sec per training step).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Workload (config.workload, identical on both arms): BASELINE.json configs[1] -- 1D Burgers, [2,20x8,1] tanh MLP,
 N_f = 100 000 collocation points per GPU (+ N_u = 100 data points), one Adam training step = fused loss/gradient
@@ -518,7 +518,14 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true")
     ap.add_argument("--no-cfg5", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (loss.npy, weights.npy, float64) to DIR, so that two builds "
+                         "can be compared output for output on the same seeded inputs")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 implementation")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -605,6 +612,8 @@ def main():
         barrier()
         launches = p.launch_count() - l0          # kernels of this library launched inside the timed region
         wall = time.perf_counter() - t_wall0
+        # read back before the untimed steps below move the weights on
+        dumped = {"loss": np.array([p.last_loss()]), "weights": p.get_weights()} if args.dump_outputs else None
         # keep the sampler alive for at least ~1.5 s of load so that it sees clocks under load; the same (fixed) number of
         # extra steps on every rank -- ranks MUST execute the same number of exchanges
         extra = int(max(0.0, 1.5 - wall) / max(wall / args.steps, 1e-5)) + 1
@@ -718,6 +727,10 @@ def main():
             line["cpu_baseline"] = cpu
         if extras is not None:
             line["extras"] = extras
+        if dumped is not None:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, arr in dumped.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), arr.astype(np.float64))
         print(json.dumps(line), flush=True)
     if dist is not None:
         barrier()

@@ -48,8 +48,13 @@ def load_golden(name):
 
 
 def load_reference_run():
-    """What the reference's OWN Python computed on the golden inputs (tests/golden/make_reference_fixtures.py)."""
-    return np.load(os.path.join(GOLDEN, "reference_run.npz"))
+    """What the reference's OWN Python computed on the golden inputs (tests/golden/make_reference_fixtures.py), kept in two
+    files so that each stays under 1 MB: the Schrodinger arrays (nls_*) in reference_run_nls.npz, the rest in reference_run.npz."""
+    run = {}
+    for name in ("reference_run", "reference_run_nls"):
+        with np.load(os.path.join(GOLDEN, name + ".npz")) as f:
+            run.update({k: f[k] for k in f.files})
+    return run
 
 
 def assert_matches_reference_run(loss, grad, loss_key, grad_key, tol=1e-10):

@@ -2,7 +2,7 @@
 reference solution burgers_shock.mat): the full evaluation grid and the default training sets of
 1d-burgers/inf_cont_burgers.py (N_u=100, N_f=10000, np.random.seed(1234)), produced by OUR prep_data restatement.
 Also runs the reference's default schedule with the CPU oracle and stores its loss curve / final error.
-    PYTHONPATH=/root/repo python tests/golden/make_accuracy_fixture.py"""
+    PYTHONPATH=. python tests/golden/make_accuracy_fixture.py"""
 import os, sys, time
 import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -10,9 +10,10 @@ sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "pinns-tf2.0_b20
 import burgersutil
 from oracle import reference_port as rp
 from neuralnetwork import _glorot_normal
+REF = os.environ.get("PINN_REFERENCE_DIR") or sys.exit("set PINN_REFERENCE_DIR to a checkout of the original PINNs-TF2.0 project")
 np.random.seed(1234)
 x, t, X, T, Exact_u, X_star, u_star, X_u, u, X_f, ub, lb = burgersutil.prep_data(
-    "/root/reference/1d-burgers/data/burgers_shock.mat", 100, 10000, noise=0.0)
+    os.path.join(REF, "1d-burgers", "data", "burgers_shock.mat"), 100, 10000, noise=0.0)
 layers = [2] + [20] * 8 + [1]
 w0 = _glorot_normal(layers, np.random.default_rng(1234))
 nu = 0.01 / np.pi

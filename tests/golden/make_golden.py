@@ -1,7 +1,7 @@
 """Generate the golden parity fixtures (tests/golden/*.npz).
 
-Run in the build container (reads the reference's data files; /root/reference does not exist on the GPU box):
-    PYTHONPATH=/root/repo python tests/golden/make_golden.py
+Needs a checkout of the original project in $PINN_REFERENCE_DIR (it reads the reference's data files):
+    PYTHONPATH=. python tests/golden/make_golden.py
 
 The reference ships no golden vectors and TensorFlow 2.0 cannot be installed here (parity against TF's kernels UNPINNED), so the
 vectors come from ``oracle.reference_port`` (nested reverse-mode restatement of the reference) and every
@@ -19,7 +19,7 @@ sys.path.insert(0, ROOT)
 from oracle import reference_port as rp, taylor as ty  # noqa: E402
 
 OUT = os.environ.get("PINN_GOLDEN_OUT", os.path.dirname(os.path.abspath(__file__)))      # tests regenerate into a scratch dir
-REF = "/root/reference"
+REF = os.environ.get("PINN_REFERENCE_DIR") or sys.exit("set PINN_REFERENCE_DIR to a checkout of the original PINNs-TF2.0 project")
 
 
 def lhs(n, d, rng):

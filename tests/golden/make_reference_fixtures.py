@@ -1,9 +1,9 @@
 """Execute the REFERENCE'S OWN, UNMODIFIED Python on the golden inputs and record what it computes.
 
-    python tests/golden/make_reference_fixtures.py            # writes tests/golden/reference_run.npz
+    python tests/golden/make_reference_fixtures.py            # writes tests/golden/reference_run{,_nls}.npz
     python tests/golden/make_reference_fixtures.py --check    # recompute and compare with the committed file, write nothing
 
-Runs only in the build container (/root/reference is absent on the GPU box; the committed .npz travels instead).
+Needs a checkout of the original project in $PINN_REFERENCE_DIR (the tests read the committed .npz files instead).
 
 What runs: ``utils/neuralnetwork.py``, ``utils/custom_lbfgs.py``, ``utils/logger.py`` imported as they are, and the
 ``*InformedNN`` class of each example script, cut out of the script by line range (the scripts train at import time) and
@@ -27,7 +27,7 @@ import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
-REF = "/root/reference"
+REF = os.environ.get("PINN_REFERENCE_DIR") or sys.exit("set PINN_REFERENCE_DIR to a checkout of the original PINNs-TF2.0 project")
 TOL = 1e-13       # observed: <= 1e-16 everywhere, including the 6-iteration fixed-step L-BFGS traces
 sys.path[:0] = [os.path.join(ROOT, "oracle", "tf_emulation"), os.path.join(REF, "utils")]
 
@@ -349,17 +349,23 @@ def main():
     worst = max(dev.values())
     print("worst: %.2e; discrete-time L-BFGS phase runs in the reference: %s" % (worst, bool(out["burgers_disc_lbfgs_runs"])))
     assert worst < TOL, "the restated oracle and the reference's own code disagree"
-    path = os.path.join(HERE, "reference_run.npz")
+    # two files, each under 1 MB: the Schrodinger arrays (nls_*) apart from the rest
+    files = {os.path.join(HERE, "reference_run.npz"): {k: v for k, v in out.items() if not k.startswith("nls_")},
+             os.path.join(HERE, "reference_run_nls.npz"): {k: v for k, v in out.items() if k.startswith("nls_")}}
     if "--check" in sys.argv:
-        old = np.load(path)
-        assert sorted(old.files) == sorted(out), "fixture keys changed"
+        old = {}
+        for path in files:
+            with np.load(path) as f:
+                old.update({k: f[k] for k in f.files})
+        assert sorted(old) == sorted(out), "fixture keys changed"
         for k in out:
             if k in ("schedule_adam_losses",) or not k.startswith("schedule_"):      # the chaotic tail may differ between machines
                 assert rel(out[k], old[k]) < 1e-12 or np.array_equal(out[k], old[k]), k
         print("committed fixture reproduced")
     else:
-        np.savez_compressed(path, **{k: np.asarray(v) for k, v in out.items()})
-        print("wrote", path, os.path.getsize(path) // 1024, "KiB")
+        for path, part in files.items():
+            np.savez_compressed(path, **{k: np.asarray(v) for k, v in part.items()})
+            print("wrote", path, os.path.getsize(path) // 1024, "KiB")
 
 
 if __name__ == "__main__":

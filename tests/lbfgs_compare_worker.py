@@ -4,11 +4,12 @@ chosen so that every exit of the routine is taken: maxIter, maxEval, optimality 
 along the direction, step below tolX, f change below tolX, rejected curvature pairs, history overflow (nCorrection)."""
 import contextlib
 import io
+import os
 import sys
 
 import numpy as np
 
-ROOT, REF = sys.argv[1], "/root/reference"
+ROOT, REF = sys.argv[1], os.environ.get("PINN_REFERENCE_DIR") or sys.exit("set PINN_REFERENCE_DIR to a checkout of the original PINNs-TF2.0 project")
 sys.path[:0] = [ROOT + "/oracle/tf_emulation", REF + "/utils", ROOT]
 import tensorflow as tf                 # noqa: E402  (emulation)
 import custom_lbfgs                     # noqa: E402  (reference)

@@ -1,7 +1,7 @@
 """Worker for test_reference_pin.py::test_logger_prints_what_the_reference_logger_prints: drives the reference utils/logger.py
-(imported from /root/reference, with the TF emulation for its banner) and the mirror with the same clock and calls."""
-import sys, io, time, importlib.util, contextlib
-ROOT, REF = sys.argv[1], "/root/reference"
+(imported from the checkout in $PINN_REFERENCE_DIR, with the TF emulation for its banner) and the mirror with the same clock and calls."""
+import os, sys, io, time, importlib.util, contextlib
+ROOT, REF = sys.argv[1], os.environ.get("PINN_REFERENCE_DIR") or sys.exit("set PINN_REFERENCE_DIR to a checkout of the original PINNs-TF2.0 project")
 sys.path[:0] = [ROOT + "/oracle/tf_emulation"]
 def load(name, path):
     spec = importlib.util.spec_from_file_location(name, path); m = importlib.util.module_from_spec(spec); spec.loader.exec_module(m); return m

@@ -1,5 +1,5 @@
 """Worker for test_reference_pin.py::test_prep_data_equals_the_reference: runs the reference's own prep_data functions
-(1d-burgers/burgersutil.py, 1dcomplex-schrodinger/schrodingerutil.py imported from /root/reference; matplotlib is stubbed --
+(1d-burgers/burgersutil.py, 1dcomplex-schrodinger/schrodingerutil.py imported from $PINN_REFERENCE_DIR; matplotlib is stubbed --
 it is only imported there, never used by prep_data -- and pyDOE.lhs is the stand-in of pinns-tf2.0_b200/shims) and the
 restatements of this package from the same numpy seed; every returned array must be bit-identical."""
 import importlib.util
@@ -9,7 +9,7 @@ import types
 
 import numpy as np
 
-ROOT, REF = sys.argv[1], "/root/reference"
+ROOT, REF = sys.argv[1], os.environ.get("PINN_REFERENCE_DIR") or sys.exit("set PINN_REFERENCE_DIR to a checkout of the original PINNs-TF2.0 project")
 
 
 class _Anything(types.ModuleType):

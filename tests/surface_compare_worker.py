@@ -1,13 +1,14 @@
 """Worker for test_reference_pin.py::test_mirror_host_attributes_equal_the_reference: builds the reference NeuralNetwork (from
-/root/reference, on the TF emulation) and the mirror for the same hp and compares every host-side attribute the scripts read."""
+$PINN_REFERENCE_DIR, on the TF emulation) and the mirror for the same hp and compares every host-side attribute the scripts read."""
 import contextlib
 import importlib.util
 import io
+import os
 import sys
 
 import numpy as np
 
-ROOT, REF = sys.argv[1], "/root/reference"
+ROOT, REF = sys.argv[1], os.environ.get("PINN_REFERENCE_DIR") or sys.exit("set PINN_REFERENCE_DIR to a checkout of the original PINNs-TF2.0 project")
 
 
 def load(name, path):

@@ -17,7 +17,7 @@ class FakePinn(object):
     instances = []
 
     def __init__(self, pde, layers, lb, ub, device=0, rank=0, world=1, nccl_uid=None):
-        self.pde, self.layers, self.launches, self.events = pde, list(layers), 0, {}
+        self.pde, self.layers, self.launches, self.events, self.steps = pde, list(layers), 0, {}, 0
         self.P = sum(a * b + b for a, b in zip(layers[:-1], layers[1:])) + (2 if pde == 1 else 0)
         FakePinn.instances.append(self)
 
@@ -25,14 +25,22 @@ class FakePinn(object):
         return None
 
     set_pde_params = set_data = set_collocation = set_collocation_ptr = set_collocation_mapped = _noop
-    set_weights = set_boundary = set_irk = sync = flush_l2 = close = _noop
+    set_boundary = set_irk = sync = flush_l2 = close = _noop
+
+    def set_weights(self, w):
+        self.steps = 0
 
     def adam_step(self, lr, b1=0.9, b2=0.999, eps=1e-7, sync=True):
         self.launches += 2
+        self.steps += 1
         return 0.5 if sync else None
 
     def adam_steps(self, n, lr, b1=0.9, b2=0.999, eps=1e-7):
         self.launches += 2 * n
+        self.steps += n
+
+    def last_loss(self):
+        return 1.0 / self.steps
 
     def event_record(self, idx):
         self.events[idx] = True
@@ -58,12 +66,12 @@ class FakePinn(object):
         return 0.25, np.ones(self.P), np.zeros(3)
 
     def get_weights(self):
-        return np.ones(self.P)
+        return np.full(self.P, float(self.steps))         # Adam steps since set_weights
 
     adam_reset = _noop
 
 
-def test_bench_gpu_arm_control_flow_with_fake_backend(monkeypatch):
+def _fake_backend(monkeypatch):
     sys.path.insert(0, ROOT)
     import torch
     import pinn_cabi
@@ -74,9 +82,14 @@ def test_bench_gpu_arm_control_flow_with_fake_backend(monkeypatch):
     monkeypatch.setattr(bench, "time_reference_port", lambda n_f, steps, warmup, seed=1234, budget_s=0: (0.4, 8, 0.1, n_f))
     monkeypatch.setattr(bench, "_port_baseline", lambda kind, data, w, steps, warmup, n, what, **kw: {"value": 1e5, "unit": "points/s", "cores": 8,
                                                                                                   "kind": "port", "sample": what})
-    monkeypatch.setattr(sys, "argv", ["bench.py", "--steps", "4", "--warmup", "1"])
     for k in ("RANK", "LOCAL_RANK", "WORLD_SIZE"):
         monkeypatch.delenv(k, raising=False)
+    return bench
+
+
+def test_bench_gpu_arm_control_flow_with_fake_backend(monkeypatch):
+    bench = _fake_backend(monkeypatch)
+    monkeypatch.setattr(sys, "argv", ["bench.py", "--steps", "4", "--warmup", "1"])
     buf = io.StringIO()
     with redirect_stdout(buf):
         bench.main()
@@ -104,6 +117,20 @@ def test_bench_gpu_arm_control_flow_with_fake_backend(monkeypatch):
         assert d["extras"][k]["cpu_baseline"]["kind"] == "port"
     assert d["extras"]["schrodinger"]["roofline"]["bound"] == "tensor"
     assert d["cpu_baseline"]["kind"] == "port" and d["cpu_baseline"]["cores"] == 8
+
+
+def test_bench_dump_outputs_are_those_of_the_last_timed_step(monkeypatch, tmp_path):
+    """--dump-outputs writes the loss and the weights as they stand after the last timed step (3 warm-up + 5 timed Adam steps),
+    not after the untimed steps that follow."""
+    bench = _fake_backend(monkeypatch)
+    out = tmp_path / "out"
+    monkeypatch.setattr(sys, "argv", ["bench.py", "--steps", "5", "--warmup", "3", "--no-extras", "--no-cpu-baseline",
+                                      "--dump-outputs", str(out)])
+    with redirect_stdout(io.StringIO()):
+        bench.main()
+    assert sorted(os.listdir(out)) == ["loss.npy", "weights.npy"]
+    loss, w = np.load(out / "loss.npy"), np.load(out / "weights.npy")
+    assert loss.dtype == w.dtype == np.float64 and loss.tolist() == [1.0 / 8] and w.shape == (3021,) and np.all(w == 8.0)
 
 
 def _launch_two(extra_args, tmp_path):

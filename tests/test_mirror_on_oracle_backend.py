@@ -4,9 +4,9 @@ no CPU path), so what is under test is everything above the C ABI: PDE recogniti
 their logger traffic, lazy losses, the flat-parameter bridge incl. lambda_1/lambda_2, the L-BFGS wrapper's arguments and
 return values, predict()/get_params() shapes.
 
-In the build container the classes are the reference's OWN class statements, cut out of its scripts and executed verbatim on
-the mirror; the results must equal tests/golden/reference_run.npz -- what the same class code produced on the emulated
-TensorFlow.  A portable variant with reference-style subclasses runs everywhere."""
+With a checkout of the original project (PINN_REFERENCE_DIR) the classes are the reference's OWN class statements, cut out
+of its scripts and executed verbatim on the mirror; the results must equal tests/golden/reference_run.npz -- what the same
+class code produced on the emulated TensorFlow.  A portable variant with reference-style subclasses runs everywhere."""
 import ast
 import importlib.util
 import io
@@ -20,7 +20,7 @@ import pytest
 
 from conftest import PKG, ROOT, load_golden, load_reference_run
 
-REF = "/root/reference"
+REF = os.environ.get("PINN_REFERENCE_DIR", "")      # a checkout of the original project, if any
 sys.path.insert(0, os.path.join(PKG, "shims"))
 
 
@@ -83,7 +83,7 @@ def fmt4(values):
     return np.array([float("%.4e" % v) for v in values])
 
 
-needs_ref = pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout only exists in the build container")
+needs_ref = pytest.mark.skipif(not os.path.isdir(REF), reason="needs a checkout of the original PINNs-TF2.0 project (set PINN_REFERENCE_DIR)")
 
 
 @needs_ref

@@ -1,6 +1,6 @@
 """CPU: the host-side mirror of the reference's Python surface (SURVEY 8(b)) up to the GPU boundary:
 module/symbol names, Struct semantics, hp parsing, flat sizes, PDE recognition, data preparation, and -- when the
-reference checkout is present (build container only) -- the UNMODIFIED inf_cont_burgers.py loading on our modules
+reference checkout is given (PINN_REFERENCE_DIR) -- the UNMODIFIED inf_cont_burgers.py loading on our modules
 through run_reference_script.py until it needs the GPU."""
 import os
 import subprocess
@@ -9,9 +9,9 @@ import sys
 import numpy as np
 import pytest
 
-from conftest import PKG, ROOT
+from conftest import PKG, ROOT, load_golden
 
-REF = "/root/reference"
+REF = os.environ.get("PINN_REFERENCE_DIR", "")      # a checkout of the original project, if any
 HP = {"N_u": 100, "N_f": 1000, "layers": [2] + [20] * 8 + [1], "tf_epochs": 3, "tf_lr": 0.03, "tf_b1": 0.9, "tf_eps": None,
       "nt_epochs": 4, "nt_lr": 0.8, "nt_ncorr": 50, "log_frequency": 10}
 
@@ -36,10 +36,18 @@ def test_struct_and_lbfgs_contract():
     assert s.anything == 0 and s.maxIter == 0
     assert lbfgs(lambda x: (0.0, x), np.zeros(3), s, Struct(), True, None) is None      # custom_lbfgs.py:43-44
     s.maxIter = 5
-    # a foreign closure runs on the stand-alone DEVICE optimiser: without a GPU that fails loudly (no host fallback)
     import pinn_cabi
-    with pytest.raises(pinn_cabi.PinnError, match="no CPU fallback"):
-        lbfgs(lambda x: (0.0, x), np.zeros(3), s, Struct(), True, None)
+    import torch
+    if not torch.cuda.is_available():
+        # a foreign closure runs on the stand-alone DEVICE optimiser: without a GPU that fails loudly (no host fallback)
+        with pytest.raises(pinn_cabi.PinnError, match="no CPU fallback"):
+            lbfgs(lambda x: (0.0, x), np.zeros(3), s, Struct(), True, None)
+    else:
+        # with one it runs there: a zero gradient at the start is optimal at once, (x, f_hist) only (custom_lbfgs.py:73-76)
+        state = Struct()
+        ret = lbfgs(lambda x: (0.0, x), np.zeros(3), s, state, True, None)
+        assert len(ret) == 2 and state.stop_reason == "initial optimality"
+        assert np.array_equal(np.asarray(ret[0]), np.zeros(3))
 
 
 def test_network_construction_and_pde_recognition(capsys):
@@ -69,12 +77,26 @@ def test_network_construction_and_pde_recognition(capsys):
             net.fit(np.zeros((5, 2)), np.zeros((5, 1)))
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout only exists in the build container")
-def test_prep_data_shapes_against_reference_files():
+@pytest.fixture()
+def burgers_shock_mat(tmp_path):
+    """The reference's 1d-burgers/data/burgers_shock.mat (x: 256, t: 100, usol: 256 x 100), rebuilt from the evaluation grid
+    prep_data made of it, which tests/golden/burgers_accuracy.npz stores (in float32)."""
+    import scipy.io
+    g = load_golden("burgers_accuracy")
+    X_star, u_star = g["X_star"].astype(np.float64), g["u_star"].astype(np.float64)
+    x, t = X_star[:256, 0], X_star[::256, 1]
+    X, T = np.meshgrid(x, t)
+    assert np.array_equal(X_star, np.hstack((X.flatten()[:, None], T.flatten()[:, None])))
+    path = str(tmp_path / "burgers_shock.mat")
+    scipy.io.savemat(path, {"x": x[:, None], "t": t[:, None], "usol": u_star.reshape(100, 256).T})
+    return path
+
+
+def test_prep_data_shapes_against_reference_files(burgers_shock_mat):
     sys.path.insert(0, os.path.join(PKG, "1d-burgers"))
     import burgersutil
     np.random.seed(1234)
-    out = burgersutil.prep_data(os.path.join(REF, "1d-burgers", "data", "burgers_shock.mat"), 100, 1000, noise=0.0)
+    out = burgersutil.prep_data(burgers_shock_mat, 100, 1000, noise=0.0)
     x, t, X, T, Exact_u, X_star, u_star, X_u, u, X_f, ub, lb = out
     assert X_star.shape == (25600, 2) and X_u.shape == (100, 2) and u.shape == (100, 1) and X_f.shape == (1000, 2)
     assert np.allclose(lb, [-1, 0]) and np.allclose(ub, [1, 0.99])
@@ -84,11 +106,11 @@ def test_prep_data_shapes_against_reference_files():
         assert sorted(np.clip(strata, 0, 999)) == list(range(1000))
     # every training point is an initial/boundary point (burgersutil.py:104-118)
     assert np.all((X_u[:, 1] == 0) | (np.abs(X_u[:, 0]) == 1))
-    ide = burgersutil.prep_data(os.path.join(REF, "1d-burgers", "data", "burgers_shock.mat"), 2000, noise=0.01)
+    ide = burgersutil.prep_data(burgers_shock_mat, 2000, noise=0.01)
     assert ide[7].shape == (2000, 2) and len(ide) == 11
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout only exists in the build container")
+@pytest.mark.skipif(not os.path.isdir(REF), reason="needs a checkout of the original PINNs-TF2.0 project (set PINN_REFERENCE_DIR)")
 def test_unmodified_reference_script_runs_up_to_the_gpu_boundary():
     import torch
     if torch.cuda.is_available():
@@ -100,7 +122,7 @@ def test_unmodified_reference_script_runs_up_to_the_gpu_boundary():
     assert "no CUDA device" in out and r.returncode != 0                # and it stops exactly at the GPU boundary
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout only exists in the build container")
+@pytest.mark.skipif(not os.path.isdir(REF), reason="needs a checkout of the original PINNs-TF2.0 project (set PINN_REFERENCE_DIR)")
 def test_indentation_normaliser_repairs_ide_cont_and_leaves_good_scripts_alone():
     import ast
     sys.path.insert(0, PKG)
@@ -121,7 +143,7 @@ def test_indentation_normaliser_repairs_ide_cont_and_leaves_good_scripts_alone()
         assert ast.dump(ast.parse(r.normalise_indentation(s0))) == ast.dump(ast.parse(s0))
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout only exists in the build container")
+@pytest.mark.skipif(not os.path.isdir(REF), reason="needs a checkout of the original PINNs-TF2.0 project (set PINN_REFERENCE_DIR)")
 @pytest.mark.parametrize("script", ["1d-burgers/ide_cont_burgers.py", "1dcomplex-schrodinger/inf_cont_schrodinger.py",
                                     "1d-burgers/inf_disc_burgers.py"])
 def test_other_reference_scripts_reach_the_gpu_boundary(script):
@@ -134,8 +156,7 @@ def test_other_reference_scripts_reach_the_gpu_boundary(script):
     assert "Training started" in out and "no CUDA device" in out and r.returncode != 0
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout only exists in the build container")
-def test_result_artefacts_hp_json_and_fields(tmp_path, monkeypatch):
+def test_result_artefacts_hp_json_and_fields(tmp_path, monkeypatch, burgers_shock_mat):
     """SURVEY 8(f)3: the plot_* helpers leave <save_path>/results/<timestamp>-<script>/{hp.json, fields.npz} behind, with or
     without matplotlib (reference: utils/plotting.py:8-16, burgersutil.py:132-203)."""
     import json
@@ -147,8 +168,7 @@ def test_result_artefacts_hp_json_and_fields(tmp_path, monkeypatch):
     sys.path.insert(0, os.path.join(PKG, "1d-burgers"))
     burgersutil = importlib.import_module("burgersutil")
     np.random.seed(0)
-    x, t, X, T, Exact_u, X_star, u_star, X_u, u_tr, X_f, ub, lb = burgersutil.prep_data(
-        os.path.join(REF, "1d-burgers", "data", "burgers_shock.mat"), 50, 500)
+    x, t, X, T, Exact_u, X_star, u_star, X_u, u_tr, X_f, ub, lb = burgersutil.prep_data(burgers_shock_mat, 50, 500)
     hp = {"N_u": 50, "layers": [2, 20, 1], "tf_eps": None, "np_value": np.float64(0.5)}
     out = burgersutil.plot_inf_cont_results(X_star, u_star.flatten() * 1.01, X_u, u_tr, Exact_u, X, T, x, t,
                                             save_path="1d-burgers", save_hp=hp)

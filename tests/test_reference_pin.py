@@ -4,7 +4,7 @@ tests/golden/reference_run.npz was produced by tests/golden/make_reference_fixtu
 utils/neuralnetwork.py, utils/custom_lbfgs.py, utils/logger.py and the *InformedNN classes of its scripts, executed in the
 build container on the TF-2.0 API emulation of oracle/tf_emulation (TensorFlow itself cannot be installed).  Here:
   * the committed reference run equals the oracle's golden values (the ones every GPU parity test compares against);
-  * where /root/reference exists, the run is repeated live and must reproduce the committed file;
+  * where a checkout of the original project is given (PINN_REFERENCE_DIR), the run is repeated live and must reproduce the committed file;
   * the emulation's tape/Keras/Adam semantics are unit-tested against TensorFlow's documented behaviour.
 """
 import os
@@ -14,9 +14,9 @@ import sys
 import numpy as np
 import pytest
 
-from conftest import ROOT, load_golden
+from conftest import ROOT, load_golden, load_reference_run
 
-REF = "/root/reference"
+REF = os.environ.get("PINN_REFERENCE_DIR", "")      # a checkout of the original project, if any
 TOL = 1e-13
 
 
@@ -26,7 +26,7 @@ def _rel(a, b):
 
 
 def _ref_run():
-    return np.load(os.path.join(ROOT, "tests", "golden", "reference_run.npz"))
+    return load_reference_run()
 
 
 def test_reference_run_equals_oracle_golden_burgers_inference():
@@ -95,7 +95,7 @@ def test_reference_run_equals_oracle_golden_discrete_time_identification():
     assert _rel(r["burgers_ide_disc_fit_w"], tr.x_eval[-1]) <= 1e-12
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout only exists in the build container")
+@pytest.mark.skipif(not os.path.isdir(REF), reason="needs a checkout of the original PINNs-TF2.0 project (set PINN_REFERENCE_DIR)")
 def test_reference_sources_reproduce_the_committed_run():
     r = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "golden", "make_reference_fixtures.py"), "--check"],
                        capture_output=True, text=True, timeout=900, cwd="/tmp")
@@ -234,7 +234,7 @@ def test_reference_default_schedule_run():
     assert _rel(r["schedule_w"], a["oracle_w"]) <= 0.05
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout only exists in the build container")
+@pytest.mark.skipif(not os.path.isdir(REF), reason="needs a checkout of the original PINNs-TF2.0 project (set PINN_REFERENCE_DIR)")
 def test_logger_prints_what_the_reference_logger_prints():
     """SURVEY 8(a) a11: with the same clock, the mirror's Logger emits the reference Logger's lines character for character
     (hyper-parameter dump, epoch lines with truncated tenths, `:.4e` losses, end line); only the version banner differs."""
@@ -243,7 +243,7 @@ def test_logger_prints_what_the_reference_logger_prints():
     assert r.returncode == 0 and "logger output identical" in r.stdout, r.stdout[-3000:] + r.stderr[-2000:]
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout only exists in the build container")
+@pytest.mark.skipif(not os.path.isdir(REF), reason="needs a checkout of the original PINNs-TF2.0 project (set PINN_REFERENCE_DIR)")
 def test_mirror_host_attributes_equal_the_reference():
     """sizes_w / sizes_b (incl. the uniform-width assumption, quirk Q7), nt_config, tf_epochs, dtype, get_params and the
     custom_lbfgs module surface of the mirror equal those of the reference classes built from the same hp."""
@@ -252,7 +252,7 @@ def test_mirror_host_attributes_equal_the_reference():
     assert r.returncode == 0 and "host attributes identical" in r.stdout, r.stdout[-3000:] + r.stderr[-3000:]
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout only exists in the build container")
+@pytest.mark.skipif(not os.path.isdir(REF), reason="needs a checkout of the original PINNs-TF2.0 project (set PINN_REFERENCE_DIR)")
 def test_prep_data_equals_the_reference():
     """SURVEY 8(f)1: every array returned by the package's prep_data restatements (Burgers inference / identification /
     discrete-time inference, Schrodinger) is bit-identical to what the reference's own prep_data returns from the same seed."""
@@ -261,7 +261,7 @@ def test_prep_data_equals_the_reference():
     assert r.returncode == 0 and "prep_data identical" in r.stdout, r.stdout[-3000:] + r.stderr[-3000:]
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout only exists in the build container")
+@pytest.mark.skipif(not os.path.isdir(REF), reason="needs a checkout of the original PINNs-TF2.0 project (set PINN_REFERENCE_DIR)")
 def test_unmodified_reference_script_runs_end_to_end_on_the_emulation(tmp_path):
     """oracle/run_reference_on_emulation.py: the whole inf_cont_burgers.py (data prep, model, fit, predict, error, result
     directory) executes on the CPU with a small hp.json; its printed log has the reference Logger's shape."""
@@ -298,7 +298,7 @@ def test_gpu_tests_reference_run_keys_exist():
         assert_matches_reference_run(float(g["loss"]) * (1 + 1e-8), g["grad"], "burgers_disc_loss", "burgers_disc_grad")
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout only exists in the build container")
+@pytest.mark.skipif(not os.path.isdir(REF), reason="needs a checkout of the original PINNs-TF2.0 project (set PINN_REFERENCE_DIR)")
 def test_lbfgs_control_flow_equals_the_reference():
     """Every exit of the reference's lbfgs() (maxIter, maxEval, optimality at the start / later, no progress, step below tolX,
     f change below tolX) plus rejected curvature pairs and history overflow: evaluation points, f history, returned x, logged
@@ -310,7 +310,7 @@ def test_lbfgs_control_flow_equals_the_reference():
     assert "reference raises UnboundLocalError" in r.stdout
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout only exists in the build container")
+@pytest.mark.skipif(not os.path.isdir(REF), reason="needs a checkout of the original PINNs-TF2.0 project (set PINN_REFERENCE_DIR)")
 def test_golden_fixtures_are_reproduced_by_their_generator(tmp_path):
     """tests/golden/make_golden.py (committed with the fixtures it made) regenerates every array of the five problem fixtures
     exactly; the generator reads only the reference's data files and the oracle."""
